@@ -44,7 +44,16 @@ def parse():
     p.add_argument('--no-extras', action='store_true', help='skip extra.bert_large / extra.allreduce_busbw / extra.checks')
     p.add_argument('--sizes', default=None, help='allreduce sweep: comma separated byte sizes')
     p.add_argument('--dtype', default='fp32', help='allreduce sweep dtype: fp32|bf16|fp16')
-    return p.parse_args()
+    p.add_argument('--dump-outputs', default=None, metavar='DIR',
+                   help='after the timed steps, write what the last timed training step computed (loss, and a fixed sample of '
+                        'the updated parameters and of the reduced gradients) as DIR/<name>.npy, to compare two builds; '
+                        'inputs are seeded, and resnet50 without --parity computes bit-identical outputs run to run')
+    args = p.parse_args()
+    if args.steps < 1:
+        p.error('--steps must be at least 1')
+    if args.dump_outputs and (args.impl != 'ours' or args.bench != 'train'):
+        p.error('--dump-outputs applies to the training benchmark of this implementation')
+    return args
 
 
 class ClockSampler:
@@ -189,15 +198,41 @@ def build_model(args, torch):
     return model, make_batch, step_fn, bs, seq, 'samples/sec'
 
 
-def _time_train(args, model_name, steps, warmup, hvd, torch, sample_clocks):
+DUMP_SAMPLE = 1 << 22  # elements per sampled output: 16 MiB of float32 each, well under 64 MiB for all dumped arrays
+
+
+def _reduced_grad(opt, p, torch):
+    """p's gradient as the optimizer applied it: a bucket reduced in a wire dtype (--bucket-wire-dtype) keeps the reduced
+    values in its bf16 / fp16 shadow, which the fused update reads directly, so p.grad still holds the local gradient."""
+    bucket = getattr(opt, '_p_to_bucket', {}).get(p)
+    if bucket is not None and bucket.get('shadow') is not None:
+        return bucket['shadow_views'][p]
+    return p.grad if p.grad is not None else torch.zeros_like(p)
+
+
+def _step_outputs(model, opt, loss, torch):
+    """What a caller of the training step holds after it: the loss, the updated parameters and the reduced gradients.
+    Parameters and gradients are flattened in model.parameters() order and sampled at fixed, seeded positions."""
+    params = torch.cat([p.detach().float().reshape(-1) for p in model.parameters()])
+    grads = torch.cat([_reduced_grad(opt, p, torch).detach().float().reshape(-1) for p in model.parameters()])
+    n = params.numel()
+    if n > DUMP_SAMPLE:
+        idx = torch.randint(n, (DUMP_SAMPLE,), generator=torch.Generator().manual_seed(0)).sort().values.to(params.device)
+        params, grads = params[idx], grads[idx]
+    return {'loss': loss.detach().float().reshape(()).cpu().numpy(), 'params': params.cpu().numpy(), 'grads': grads.cpu().numpy()}
+
+
+def _time_train(args, model_name, steps, warmup, hvd, torch, sample_clocks, keep_outputs=False):
     """One training configuration: device-timed arm (inputs resident) and end-to-end arm (per-step pinned H2D input copy +
-    D2H loss read).  Returns a dict; frees the model before returning."""
+    D2H loss read).  Returns a dict (with keep_outputs, under 'outputs' what the last device-timed step computed); frees
+    the model before returning."""
     from horovod_b200.data import DevicePrefetcher
     rank, size, local_rank = hvd.rank(), hvd.size(), hvd.local_rank()
     margs = argparse.Namespace(**vars(args))
     margs.model = model_name
     if model_name != args.model:
         margs.batch_size, margs.seq_len = None, None
+    torch.manual_seed(0)  # same weights and batch on every run with the same arguments, so runs can be compared output for output
     model, make_batch, step_fn, bs, seq, unit = build_model(margs, torch)
     use_bf16 = not args.fp32
     eager = args.no_cuda_graph or args.parity
@@ -286,8 +321,9 @@ def _time_train(args, model_name, steps, warmup, hvd, torch, sample_clocks):
     sampler = ClockSampler(local_rank) if (rank == 0 and sample_clocks) else None
     if sampler:
         sampler.start()
-    ms, launches, _ = timed(steps, e2e=False)
+    ms, launches, last = timed(steps, e2e=False)
     clocks = sampler.stop() if sampler else None
+    outputs = _step_outputs(model, opt, last, torch) if keep_outputs else None
     for _ in range(2):
         graphed(*tuple(t.cuda(non_blocking=True) for t in host_batch))
     e2e_ms, _, last_loss = timed(steps, e2e=True)
@@ -307,7 +343,7 @@ def _time_train(args, model_name, steps, warmup, hvd, torch, sample_clocks):
         'global_batch': global_batch, 'per_gpu_batch': bs, 'seq_len': seq, 'params_identical_across_ranks': params_identical,
         'cuda_graph': bool(graphed.captured), 'cuda_graph_fallback': graphed.fallback_reason,
         'allreduce_in_graph': bool(graphed.comm_in_graph), 'gradient_buckets': len(getattr(opt, '_buckets', [])),
-        'optimizer': 'SGD(momentum=0.9)' if model_name == 'resnet50' else 'AdamW',
+        'optimizer': 'SGD(momentum=0.9)' if model_name == 'resnet50' else 'AdamW', 'outputs': outputs,
     }
     del graphed, opt, base_opt, model, dev_batch, host_batch
     import gc
@@ -445,12 +481,23 @@ def train_bench(args):
     hvd.init()
     rank, size = hvd.rank(), hvd.size()
     torch.cuda.set_device(hvd.local_rank())
-    torch.backends.cudnn.benchmark = True
+    # convolution algorithms from cuDNN's heuristics, deterministic ones only, so that two runs with the same arguments
+    # compute the same steps: benchmark mode picks algorithms by timing them, and the pick differs from run to run.  It is
+    # not faster here (ResNet-50, batch 64, bf16, one B200 at 1000 W, alternating runs: 4229 / 4236 img/s benchmark mode,
+    # 4281 / 4412 img/s heuristics + deterministic).  --parity keeps the stock benchmark's benchmark mode.
+    torch.backends.cudnn.benchmark = args.parity
+    torch.backends.cudnn.deterministic = not args.parity
     torch.backends.cuda.matmul.allow_tf32 = not args.parity
     torch.backends.cudnn.allow_tf32 = not args.parity
     if args.parity:
         args.fp32 = True  # the stock reference benchmark: fp32, eager hooks, unfused optimizer, batch 64
-    main = _time_train(args, args.model, args.steps, args.warmup, hvd, torch, sample_clocks=True)
+    main = _time_train(args, args.model, args.steps, args.warmup, hvd, torch, sample_clocks=True,
+                       keep_outputs=bool(args.dump_outputs) and rank == 0)
+    if main['outputs'] is not None:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in main['outputs'].items():
+            np.save(os.path.join(args.dump_outputs, name + '.npy'), a)
     extra = {}
     if not args.no_extras:
         try:
@@ -482,7 +529,9 @@ def train_bench(args):
                        'seq_len': main['seq_len'], 'parallelism': f'dp{size}', 'optimizer': main['optimizer'],
                        'fused_optimizer': not (args.no_fused_optimizer or args.parity), 'grad_dtype': 'fp32',
                        'bucket_wire_dtype': args.bucket_wire_dtype or 'fp32', 'bucket_cap_mb': args.bucket_cap_mb,
-                       'parity_mode': bool(args.parity), 'cuda_graph': main['cuda_graph'], 'cuda_graph_fallback': main['cuda_graph_fallback'],
+                       'parity_mode': bool(args.parity),
+                       'cudnn': {'benchmark': torch.backends.cudnn.benchmark, 'deterministic': torch.backends.cudnn.deterministic},
+                       'cuda_graph': main['cuda_graph'], 'cuda_graph_fallback': main['cuda_graph_fallback'],
                        'allreduce_in_graph': main['allreduce_in_graph'], 'gradient_buckets': main['gradient_buckets'],
                        'l2': 'per-step working set (activations + 100+ MB of gradients) exceeds the 126 MB L2; no explicit flush',
                        'gpu_backend': hvd.gpu_backend_info(), 'tunables': hvd.tunable_params()},

@@ -151,8 +151,6 @@ def test_sim_allgather_exchange():
         assert torch.equal(outs[r], ref)
 
 
-@pytest.mark.skipif(__import__('os').environ.get('HVD_RUN_NEW_GPU_TESTS', '0') != '1',
-                    reason='TMA exchange kernel: written after the GPU budget of round 1 was spent; HVD_RUN_NEW_GPU_TESTS=1')
 def test_sim_allgather_exchange_tma_variant():
     """The cp.async.bulk (UBLKCP) variant of the exchange kernel: ragged sizes (16 B-aligned bulk part + byte tail) and an
     unaligned destination (falls back to the vector path inside the same kernel).  Runs in a subprocess because the
@@ -183,8 +181,6 @@ def test_sim_allgather_exchange_tma_variant():
     assert p.returncode == 0 and 'TMA EXCHANGE OK' in p.stdout.decode(), p.stdout.decode()[-3000:]
 
 
-@pytest.mark.skipif(__import__('os').environ.get('HVD_RUN_NEW_GPU_TESTS', '0') != '1',
-                    reason='software-pipelined allreduce: written after the GPU budget of round 1 was spent; HVD_RUN_NEW_GPU_TESTS=1')
 @pytest.mark.parametrize("slots", ["2", "16"])
 def test_pipelined_allreduce_variant_in_simulation(slots):
     """kPipelined (role-specialised CTAs, chunk ring in the symmetric buffer, packed / reduced / unpack_done counters) with

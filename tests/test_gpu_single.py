@@ -105,3 +105,28 @@ def test_graphed_step_matches_eager(hvd, fused):
 def test_smoke_entry():
     import __graft_entry__ as g
     g.smoke()
+
+
+def test_bench_dump_outputs_are_reproducible(tmp_path):
+    """`bench.py --dump-outputs DIR` writes the last timed step's loss / parameter sample / gradient sample as float32 .npy,
+    under 64 MB in all, and a second run with the same arguments writes the same arrays bit for bit."""
+    import os
+    import subprocess
+    import sys
+    import numpy as np
+    from conftest import REPO
+    dumps = []
+    for run in ('a', 'b'):
+        d = tmp_path / run
+        r = subprocess.run([sys.executable, os.path.join(REPO, 'bench.py'), '--gpus', '1', '--steps', '2', '--warmup', '0',
+                            '--no-extras', '--dump-outputs', str(d)], cwd=REPO, capture_output=True, text=True, timeout=600)
+        assert r.returncode == 0, r.stderr[-3000:]
+        assert sorted(os.listdir(d)) == ['grads.npy', 'loss.npy', 'params.npy']
+        assert sum(f.stat().st_size for f in d.iterdir()) < 64 << 20
+        dumps.append({n: np.load(d / (n + '.npy')) for n in ('loss', 'params', 'grads')})
+    a, b = dumps
+    assert a['loss'].shape == () and a['params'].shape == a['grads'].shape == (1 << 22,)
+    assert all(x.dtype == np.float32 and np.isfinite(x).all() for x in a.values())
+    assert np.abs(a['grads']).max() > 0
+    for n in a:
+        assert np.array_equal(a[n], b[n]), n

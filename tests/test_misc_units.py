@@ -135,6 +135,21 @@ def test_bench_reference_arm_reports_unavailable():
         assert 'mpi_lib_v2' in rec['unavailable'] or 'does not build offline' in rec['unavailable']
 
 
+def test_bench_rejects_bad_arguments():
+    """bench.py refuses a run with no timed step, and --dump-outputs outside the training benchmark of this library."""
+    import os
+    import subprocess
+    import sys
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    for extra, msg in ((['--steps', '0'], '--steps must be at least 1'),
+                       (['--dump-outputs', 'out', '--impl', 'reference'], '--dump-outputs applies to'),
+                       (['--dump-outputs', 'out', '--bench', 'allreduce'], '--dump-outputs applies to')):
+        r = subprocess.run([sys.executable, os.path.join(root, 'bench.py')] + extra, cwd=root, capture_output=True, text=True,
+                           timeout=120)
+        assert r.returncode == 2 and msg in r.stderr, (extra, r.stderr[-2000:])
+        assert not os.path.exists(os.path.join(root, 'out'))
+
+
 def test_every_hvd_knob_is_documented():
     """docs/knobs.md lists every HVD_* environment variable the sources read."""
     import os
